@@ -3,7 +3,7 @@
 roofline).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--configs 2,3,4,5] [--kernels-only]
+                    [--configs 2,3,4,5] [--kernels-only] [--dump-outputs DIR]
 
 Headline workload (SURVEY 8d config 2): Morlet(6) CWT of a synthetic linear chirp, N = 2^20,
 256 scales (s0=2, dj=1/16, J=255), fp64.  One "step" = one full transform of one signal (forward
@@ -16,6 +16,10 @@ its own `e2e`, `roofline` and `cpu_baseline`; under torchrun also the two sharde
 SURVEY 8e (config 5 channels over ranks with the NCCL gather of the spectra inside the timed
 region; config 2 scales over ranks, strong scaling).  `--configs 2` restricts the run to the
 headline.  See DESIGN.md "Measurement" for every field.
+
+`--dump-outputs DIR` writes, after the timed steps, what the headline transform computed in its
+last step (see `dump_config2`), so that two builds can be compared output for output: the
+inputs depend only on the arguments.
 """
 import argparse
 import hashlib
@@ -349,6 +353,24 @@ def config2_description():
 # ---------------------------------------------------------------------------------------------
 # config 2 (headline)
 # ---------------------------------------------------------------------------------------------
+DUMP_COLUMNS = 8192
+
+
+def dump_config2(out_dir, eng, n_scales, n):
+    """The outputs of the resident transform as a caller fetches them (`Engine.get_w`,
+    `Engine.signal_fft`), as float64 .npy files: W at every scale for DUMP_COLUMNS time
+    indices drawn once from RandomState(0), sorted (W_real, W_imag: 32 MiB of the 4 GiB), and
+    the signal spectrum returned beside it (fft_real, fft_imag)."""
+    os.makedirs(out_dir, exist_ok=True)
+    cols = np.sort(np.random.RandomState(0).choice(n, min(n, DUMP_COLUMNS), replace=False))
+    W = eng.get_w(n_scales, n)
+    Ws = W[:, cols]
+    del W
+    fft = eng.signal_fft()
+    for name, a in (("W_real", Ws.real), ("W_imag", Ws.imag), ("fft_real", fft.real), ("fft_imag", fft.imag)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def run_config2(args, D, eng, pycwt, _engine):
     c = wl.C2
     sj = wl.config2_scales()
@@ -372,6 +394,8 @@ def run_config2(args, D, eng, pycwt, _engine):
     D.barrier()
     clocks = sampler.stop()
     ms_max = D.max(ms)
+    if args.dump_outputs and D.rank == 0:
+        dump_config2(args.dump_outputs, eng, S, c["n"])
     value = D.world * pts / (ms_max * 1e-3)
     prof = eng.profile_last()    # per-kernel-type event times of one more (untimed, serialised) step
     eng.dev_free(dsig)
@@ -451,7 +475,7 @@ def run_config3(args, D, eng, pycwt, _engine):
     x = wl.config3_signal()
     out = {"workload": "config3: Paul(4) and DOG(2) CWT, chirp N=2^18 (float32), 128 scales, fp32 engine",
            "dtype": "f32", "metric": METRIC, "unit": UNIT}
-    steps = max(args.steps, 20)
+    steps = args.steps
     mod, kind = reference_module()
     os.environ["CWTB_PRECISION"] = "fp32"
     try:
@@ -599,13 +623,13 @@ def run_config5(args, D, eng, pycwt, _engine, comm=None):
     eng.cwt_batch_dev(dX, chunk, c["n"], c["dt"], sj, _engine.MORLET, c["f0"], _engine.F32)
     eng.bench_last(2)
     D.barrier()
-    ms = D.max(eng.bench_last(5))
+    ms = D.max(eng.bench_last(args.steps))
     launches = eng.last_launch_count()
     prof = eng.profile_last()
     eng.dev_free(dX)
     pts_chunk = chunk * S * c["n"]
-    out.update({"value": D.world * pts_chunk / (ms * 1e-3), "ms_per_step": ms, "steps": 5,
-                "step": "one 256-channel chunk (4 per GPU share)", "gpu_launches": launches * 5,
+    out.update({"value": D.world * pts_chunk / (ms * 1e-3), "ms_per_step": ms, "steps": args.steps,
+                "step": "one 256-channel chunk (4 per GPU share)", "gpu_launches": launches * args.steps,
                 "roofline": roofline_block(prof, c["n"] * 8, pts_chunk * 8 + chunk * c["n"] * 4, ms)})
     # end to end: host float32 channels in, per-channel spectra out, gathered over the ranks
     from pycwt_b200 import distributed as Dm
@@ -717,7 +741,14 @@ def main():
                     help="BASELINE.json configurations to measure (2 is always the headline)")
     ap.add_argument("--kernels-only", action="store_true",
                     help="profiling aid: time the resident-input kernels of config 2 only")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed sample of the headline transform's outputs of its last "
+                         "timed step to DIR/<name>.npy (float64, 40 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this project's transform (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,7 +1,7 @@
 """Helper of tests/test_bench_contract.py: runs bench.py's PRODUCT arm on the host-emulation
 build with a small signal, so that the assembly of the JSON line (keys, roofline, e2e, clocks)
 is exercised where no GPU is present.  The emulation has no clock, so the device-timing hooks are
-given fixed numbers; the printed throughput means nothing."""
+given fixed numbers; the printed throughput means nothing.  Extra arguments go to bench.py."""
 import os
 import sys
 
@@ -24,5 +24,5 @@ bench.wl.C2["n"] = 2 ** 12
 bench.ClockSampler = type("CS", (), {
     "__init__": lambda s, *a, **k: None, "start": lambda s: None,
     "stop": lambda s: {"sm_mhz": 1965.0, "sm_max_mhz": 1965.0, "samples": 1, "reasons": []}})
-sys.argv = ["bench.py", "--steps", "3", "--warmup", "1", "--configs", "2"]
+sys.argv = ["bench.py", "--steps", "3", "--warmup", "1", "--configs", "2"] + sys.argv[1:]
 bench.main()

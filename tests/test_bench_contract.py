@@ -38,17 +38,25 @@ def test_reference_arm_prints_one_contract_line():
     assert cb["cores"] == 1 and cb["value"] == d["value"] and cb["sample"]
 
 
+#: SHA-256 of the reference package's files at v0.3.0a22 (commit f88aec2)
+REFERENCE_SHA256 = {
+    "__init__.py": "568ec8dab26353a2167732d6756fd1efccb3e53e3c625a51de82cd247bb5b30f",
+    "wavelet.py": "12aa7178db085ce128b392b0db645d8b4c4093442a431ec2cd3469e69869fcd2",
+    "mothers.py": "500111993e025651a935de3dd5f6abd9dd4113b4fea01d981e18c46c7fe39443",
+    "helpers.py": "116395fb05b6bf227b6f2463618635c080c090d8851e06b1bf6d7760bb80759f",
+}
+
+
 def test_reference_copy_is_the_unmodified_reference():
-    """oracle/_ref/pycwt (the timing arm) is byte-identical to the reference checkout where both exist."""
+    """oracle/_ref/pycwt (the timing arm), where it was built, is byte-identical to the reference."""
     import hashlib
     from oracle import make_ref
-    src = os.path.join(make_ref.REF_ROOT, "pycwt")
-    if not (make_ref.available() and os.path.isdir(src)):
+    assert sorted(make_ref.FILES) == sorted(REFERENCE_SHA256)
+    if not make_ref.available():
         return
     for f in make_ref.FILES:
-        a = hashlib.sha256(open(os.path.join(src, f), "rb").read()).hexdigest()
         b = hashlib.sha256(open(os.path.join(make_ref.DST, "pycwt", f), "rb").read()).hexdigest()
-        assert a == b, f
+        assert b == REFERENCE_SHA256[f], f
     mod = make_ref.load()
     assert mod.__version__ == "0.3.0a22" and mod.cwt.__module__ == "pycwt.wavelet"
 
@@ -100,3 +108,23 @@ def test_product_arm_json_assembly_on_the_emulation_build():
     assert set(d["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
     assert d["e2e"]["resident"]["value"] > 0 and d["configs"] == {}
     assert rf["kernel"] == "PassBBody<double, 1, 1024>" and rf["source_hash"]
+
+
+def test_dump_outputs_are_the_headline_transform(tmp_path):
+    """--dump-outputs writes the sampled W and the signal spectrum of the timed transform (here
+    the emulation build at N = 2^12, where every column is kept) as float64 files."""
+    import numpy as np
+    import workloads as wl
+    from oracle import cwt_oracle as orc
+    from conftest import relerr
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "_bench_emu_driver.py"),
+                        "--dump-outputs", str(tmp_path)], cwd=ROOT, capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    out = {f[:-4]: np.load(os.path.join(tmp_path, f)) for f in os.listdir(tmp_path)}
+    assert sorted(out) == ["W_imag", "W_real", "fft_imag", "fft_real"]
+    assert all(a.dtype == np.float64 for a in out.values())
+    c, n = wl.C2, 2 ** 12
+    x = wl.chirp(n)
+    W, _, _, _, fft, _ = orc.cwt(x, c["dt"], c["dj"], c["s0"], c["J"], orc.Morlet(c["f0"]))
+    assert relerr(out["W_real"] + 1j * out["W_imag"], W) < 1e-10
+    assert relerr(out["fft_real"] + 1j * out["fft_imag"], fft) < 1e-10
