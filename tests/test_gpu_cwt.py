@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 from conftest import load_golden, relerr, golden_cwt_kwargs
+from _rowerr import check_rows
 from oracle import cwt_oracle as orc
 
 pytestmark = pytest.mark.gpu
@@ -138,9 +139,10 @@ def test_all_plan_classes_exercised(pycwt):
     plan = eng.last_plan(len(sj))
     assert set(plan) >= set(range(-13, -5)) and max(plan) == 16, plan   # coarse grids 2^6..2^13
     assert relerr(W, Wr) < 2e-13
-    for i, p in enumerate(plan):
-        if p < 0:
-            assert np.abs(W[i] - Wr[i]).max() < 2e-13 * np.abs(Wr).max(), (i, p)
+    # every expansion row on its own (the global maximum hides the small rows)
+    rows = [i for i, p in enumerate(plan) if p < 0]
+    err = check_rows(W[rows], Wr[rows], 1e-12, 1e-14, what="expansion rows")
+    print("expansion rows: worst row error %.2e" % err)
 
 
 def test_expansion_path_families_and_precisions(pycwt, monkeypatch):
