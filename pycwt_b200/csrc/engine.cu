@@ -806,6 +806,8 @@ static int fft_rows_small(cwtb_ctx *c, const RowsArgs<T> &a) {
 template <typename T, int SIGN, int K1, int MODE>
 static int launch_passA(cwtb_ctx *c, const PassAArgs<T> &a, int ny) {
   using B = PassABody<T, K1, MODE, SIGN>;
+  // a tile covers T2 consecutive r2 of one output row: a shorter row would launch no block at all
+  if (a.K2 % B::T2 != 0) return fail(c, CWTB_ERR_STATE, "first kernel: row length not a multiple of its tile");
   const unsigned M = a.N / ((unsigned)K1 * a.K2);
   return launch<B>(c, M * (a.K2 / B::T2), ny, a);
 }
@@ -1683,7 +1685,11 @@ static int run_job(cwtb_ctx *c, const Job &job, const T *dsig, cx<T> *Wout = nul
       // (fp32: the 512-point tile has an odd row pitch, its rows would not be 16-byte aligned)
       constexpr bool k512_ok = (Lay<T, 512, true>::PITCH * sizeof(V)) % 16 == 0;
       // 512 pays up to K' = 2^16 (measured per class: first kernel + second kernel per row)
-      const int l2k = (dense || persistent || cl.log2K > c->k2_512_max_log2 || !k512_ok) ? 10 : c->k2_band_log2;
+      // (a first kernel of K1 points covers TILE / K1 values of r2 per tile: at most 512 for rows
+      // of 512, so K1 >= 8 in fp64; K' = 2^11 under CWTB_DIRECT_MAX=10 keeps 1024)
+      const bool k1_fits_512 = (TileCfg<T>::TILE >> std::max(0, cl.log2K - 9)) <= 512;
+      const int l2k = (dense || persistent || cl.log2K > c->k2_512_max_log2 || !k512_ok || !k1_fits_512)
+                          ? 10 : c->k2_band_log2;
       a.pf_dist = c->pf_dist_a; a.K2 = 1u << l2k; a.gauss_rec = c->gauss_rec;
       PassBArgs<T> b{};
       b.Z = (const V *)Zb.p; b.out = W; b.tw = Tw<T>::get(c); b.descs = ddesc;

@@ -43,20 +43,28 @@ def test_cwt_kernels_vs_reference_fixture(emu, name):
 
 
 def test_every_pruned_class_and_dense_path(emu):
-    """Exact mode (expansion off): every pruned length 2^5..2^15 and the dense path."""
+    """Exact mode (expansion off): every pruned length 2^5..2^15 and the dense path, every row
+    on its own (tests/test_emu_exact.py: the row gates of the exact path), on a chirp in white
+    noise and on white noise alone."""
+    from test_emu_exact import GATE
     n = 2 ** 15
     t = np.arange(n) / n
-    x = np.sin(2 * np.pi * (50 * t + (n / 8) * t ** 2)) + 0.1 * np.random.RandomState(1).randn(n)
+    noise = np.random.RandomState(1).randn(n)
     sj = 2.0 * 2 ** (np.arange(0, 27) / 2.0)
-    Wr = orc.cwt(x, 1.0, wavelet=orc.Morlet(6), freqs=1 / (orc.Morlet(6).flambda() * sj))[0]
+    m = orc.Morlet(6)
     emu.set_expand_eps(0.0, 0.0)
     try:
-        W = emu.cwt(x, 1.0, sj, 0, 6.0)
-        plan = emu.last_plan(len(sj))
-        assert set(plan) >= set(range(5, 16)), plan   # single, direct (11..13), two-kernel, dense
-        assert relerr(W, Wr) < 1e-14
-        W32 = emu.cwt(x.astype(np.float32), 1.0, sj, 0, 6.0, precision=1)
-        assert relerr(W32, Wr) < 1e-5
+        for x in (np.sin(2 * np.pi * (50 * t + (n / 8) * t ** 2)) + 0.1 * noise, noise):
+            Wr = orc.cwt(x, 1.0, wavelet=m, freqs=1 / (m.flambda() * sj))[0]
+            W = emu.cwt(x, 1.0, sj, 0, 6.0)
+            plan = emu.last_plan(len(sj))
+            assert set(plan) >= set(range(5, 16)), plan   # single, direct (11..13), two-kernel, dense
+            err = check_rows(W, Wr, *GATE[0], what="fp64")
+            W32 = emu.cwt(x.astype(np.float32), 1.0, sj, 0, 6.0, precision=1)
+            Wr32 = orc.cwt(x.astype(np.float32).astype(np.float64), 1.0, wavelet=m,
+                           freqs=1 / (m.flambda() * sj))[0]
+            err32 = check_rows(W32, Wr32, *GATE[1], what="fp32")
+            print("exact rows: worst row error fp64 %.2e, fp32 %.2e" % (err, err32))
     finally:
         emu.set_expand_eps()
 

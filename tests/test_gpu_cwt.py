@@ -124,15 +124,22 @@ def test_lengths_edge_cases(pycwt, n0):
 def test_all_plan_classes_exercised(pycwt):
     """One transform that uses every pruned length 2^5..2^16 and the dense path (exact mode:
     expansion path off), then the same transform in the default mode (expansion path on)."""
-    x = chirp(2 ** 16) + 0.1 * np.random.RandomState(1).randn(2 ** 16)
+    from test_emu_exact import GATE
+    noise = np.random.RandomState(1).randn(2 ** 16)
+    x = chirp(2 ** 16) + 0.1 * noise
     Wr = orc.cwt(x, 1.0, dj=0.5, s0=2.0, J=30, wavelet=orc.Morlet(6))[0]
     eng = pycwt.default_engine()
     eng.set_expand_eps(0.0, 0.0)
     try:
-        W, sj, *_ = pycwt.cwt(x, 1.0, dj=0.5, s0=2.0, J=30, wavelet=pycwt.Morlet(6))
-        plan = eng.last_plan(len(sj))
-        assert set(plan) >= set(range(5, 17)), plan
-        assert relerr(W, Wr) < 1e-14
+        # every exact row on its own, on the chirp and on white noise alone
+        for xx, ref in ((x, Wr), (noise, None)):
+            W, sj, *_ = pycwt.cwt(xx, 1.0, dj=0.5, s0=2.0, J=30, wavelet=pycwt.Morlet(6))
+            plan = eng.last_plan(len(sj))
+            assert set(plan) >= set(range(5, 17)), plan
+            if ref is None:
+                ref = orc.cwt(xx, 1.0, dj=0.5, s0=2.0, J=30, wavelet=orc.Morlet(6))[0]
+            err = check_rows(W, ref, *GATE[0], what="exact rows")
+            print("exact rows: worst row error %.2e" % err)
     finally:
         eng.set_expand_eps()
     W, sj, *_ = pycwt.cwt(x, 1.0, dj=0.5, s0=2.0, J=30, wavelet=pycwt.Morlet(6))

@@ -17,8 +17,8 @@ import re
 
 import numpy as np
 import pytest
-import scipy.fft as sfft
 
+from _gpu_rows import fetch_rows, kernel_counts, oracle_rows, profiled
 from _rowerr import check_rows
 from oracle import cwt_oracle as orc
 
@@ -49,47 +49,9 @@ def scales(log2N):
     return 2.0 ** (np.arange(20, 4 * (log2N + 2)) / 4.0)
 
 
-def oracle_rows(x, sj, rows, mother=None):
-    """Rows `rows` of the reference transform (padded to the next power of two, dt = 1)."""
-    mo = mother or orc.Morlet(6)
-    n0 = len(x)
-    npad = orc.next_pow2(n0)
-    xh = sfft.fft(x, npad)
-    om = 2 * np.pi * sfft.fftfreq(npad, 1.0)
-    out = np.empty((len(rows), n0), dtype=np.complex128)
-    for i, j in enumerate(rows):
-        filt = np.sqrt(sj[j] * om[1] * npad) * np.conj(mo.psi_ft(sj[j] * om))
-        out[i] = sfft.ifft(xh * filt, workers=-1)[:n0]
-    return out
-
-
-def fetch_rows(e, rows, n0):
-    """Rows of the resident transform, one device-to-host copy each."""
-    out = np.empty((len(rows), n0), dtype=np.complex128)
-    for i, j in enumerate(rows):
-        e._check(e.lib.cwtb_get_w(e.h, out[i].ctypes.data, 1, int(j), 1))
-    return out
-
-
 def expand_kernels(prof, pattern=MMA):
     """{(taps, epilogue): launches} of the expansion kernels in a profile."""
-    out = {}
-    for p in prof:
-        m = pattern.search(p["name"])
-        if m:
-            key = (int(m.group(1)), int(m.group(2) or 0))
-            out[key] = out.get(key, 0) + p["launches"]
-    return out
-
-
-def profiled(e, fn):
-    """fn() between profile_begin / profile_end: (its result, the profile)."""
-    e.profile_begin()
-    try:
-        res = fn()
-    finally:
-        prof = e.profile_end()
-    return res, prof
+    return kernel_counts(prof, pattern)
 
 
 def expansion_rows(plan):
