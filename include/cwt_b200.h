@@ -227,6 +227,33 @@ int cwtb_cwt_batch(cwtb_ctx *ctx, const void *X, int x_is_f32, int n_chan,
                    int family, double param, int precision, double *power_out,
                    void *W_out);
 
+/* Batched transform with per-channel products reduced on the device while each chunk of W is
+ * resident (W itself never leaves the device).  Arguments as cwtb_cwt_batch, plus:
+ *   coi_lo, coi_hi  int64[n_scales], both or neither: columns lo_j <= n < hi_j inside the cone of
+ *                   influence (the same for every channel);
+ *   n_bands (0..8), band_weights [n_bands][n_scales];  chan_scale [n_chan] (NULL: 1);
+ *   icwt_re, icwt_im: the icwt factor dj*sqrt(dt)/(Cdelta*psi(0));  want_icwt: 0 none,
+ *                   1 real output, 2 complex output.
+ * Outputs (doubles, per channel c; pycwt/sample/simple_sample.py lines each restates):
+ *   power_out     [n_chan][n_scales]  mean_n |W|^2                          (glbl_power, :79; required)
+ *   power_coi_out [n_chan][n_scales]  mean of |W|^2 over [lo_j, hi_j), NaN if empty (with the ranges)
+ *   band_out      [n_chan][n_bands][n0]  chan_scale[c] * sum_j wt[b][j] |W[c,j,n]|^2
+ *                                     (scale_avg, :88-91, with wt = dj*dt/Cdelta/s_j in the band)
+ *   icwt_out      [n_chan][n0] (want_icwt 1) or [n_chan][n0][2] (want_icwt 2):
+ *                 factor * sum_j Re(W[c,j,n]) / sqrt(s_j)                  (iwave, :60)
+ * Every coefficient is read once, by one kernel per chunk.  With the default pipeline the column
+ * outputs of chunk k are copied to the host while chunk k+1 is transformed; page-locked output
+ * arrays (cwtb_host_alloc) make that copy asynchronous.  CWTB_ERR_UNSUPPORTED for CWTB_TABLE and
+ * for an un-padded (cwtb_set_padding(0)) length that is not a power of two. */
+int cwtb_cwt_batch_products(cwtb_ctx *ctx, const void *X, int x_is_f32, int n_chan,
+                            int64_t n0, double dt, const double *scales, int n_scales,
+                            int family, double param, int precision,
+                            const int64_t *coi_lo, const int64_t *coi_hi,
+                            int n_bands, const double *band_weights, const double *chan_scale,
+                            double icwt_re, double icwt_im, int want_icwt,
+                            double *power_out, double *power_coi_out, double *band_out,
+                            double *icwt_out);
+
 /* Device-resident variant: d_X [n_chan][n0] already on the device in the engine's real type;
  * one chunk (n_chan * n_scales rows <= 60000); W [n_chan][n_scales][n0] stays resident
  * (cwtb_w_device_ptr); power_out (may be NULL): host [n_chan][n_scales] mean |W|^2. */

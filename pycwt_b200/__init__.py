@@ -10,6 +10,7 @@ from . import helpers, mothers, wavelet  # noqa: F401  (reachable as attributes,
 from .wavelet import *  # noqa: F401,F403
 from ._engine import Engine, EngineError, default_engine, device_count  # noqa: F401
 from .resident import cwt_resident, ResidentTransform  # noqa: F401  (B200 extension, SURVEY 8f)
+from .batch import cwt_batch, BatchProducts  # noqa: F401  (B200 extension: per-channel products of a batch)
 
 __all__ = ['cwt', 'icwt', 'significance', 'xwt', 'wct', 'wct_significance',
            'mothers', 'Morlet', 'Paul', 'DOG', 'MexicanHat']

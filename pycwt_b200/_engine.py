@@ -71,6 +71,8 @@ _SIGNATURES = {
     "cwtb_mc_surrogates": (_I, [_P, ctypes.c_uint64, _I64, _I, _I64, _P]),
     "cwtb_cwt_batch": (_I, [_P, _P, _I, _I, _I64, _D, _P, _I, _I, _D, _I, _P, _P]),
     "cwtb_cwt_batch_dev": (_I, [_P, _P, _I, _I64, _D, _P, _I, _I, _D, _I, _P]),
+    "cwtb_cwt_batch_products": (_I, [_P, _P, _I, _I, _I64, _D, _P, _I, _I, _D, _I, _P, _P, _I, _P, _P,
+                                     _D, _D, _I, _P, _P, _P, _P]),
     "cwtb_comm_unique_id": (_I, [_P]),
     "cwtb_comm_init": (_I, [_P, _I, _I, _P]),
     "cwtb_comm_destroy": (_I, [_P]),
@@ -566,6 +568,60 @@ class Engine(object):
                                                 _ptr(W) if want_w else None))
             self._resident = None                   # the last chunk of channels only
         return power, W
+
+    @_locked
+    def cwt_batch_products(self, X, dt, scales, family, param, precision=F64, coi_ranges=None,
+                           band_weights=None, chan_scale=None, icwt_factor=None):
+        """Batched transform of the rows of X [C, n0] with per-channel products reduced on the
+        device (cwtb_cwt_batch_products).  coi_ranges: (lo, hi) int64 per scale; band_weights:
+        [n_bands, S]; chan_scale: C factors of the band powers; icwt_factor: real or complex
+        (the type of the icwt output).  Returns (power [C, S], power_coi [C, S] or None,
+        band [C, n_bands, n0] or None, icwt [C, n0] or None)."""
+        X = np.ascontiguousarray(X)
+        if X.dtype != np.float32:
+            X = np.ascontiguousarray(X, dtype=np.float64)
+        if X.ndim != 2:
+            raise ValueError("cwt_batch_products: X must be [channels, samples]")
+        sj = np.ascontiguousarray(scales, dtype=np.float64)
+        nch, n0 = X.shape
+        power = np.empty((nch, sj.size), dtype=np.float64)
+        lo = hi = power_coi = None
+        if coi_ranges is not None:
+            lo = np.ascontiguousarray(coi_ranges[0], dtype=np.int64)
+            hi = np.ascontiguousarray(coi_ranges[1], dtype=np.int64)
+            if lo.shape != (sj.size,) or hi.shape != (sj.size,):
+                raise ValueError("cwt_batch_products: one COI range per scale expected")
+            power_coi = np.empty((nch, sj.size), dtype=np.float64)
+        wt = band = None
+        nb = 0
+        if band_weights is not None:
+            wt = np.ascontiguousarray(band_weights, dtype=np.float64)
+            if wt.ndim != 2 or wt.shape[1] != sj.size:
+                raise ValueError("cwt_batch_products: band weights must be [n_bands, scales]")
+            nb = wt.shape[0]
+            if nb > 0:
+                band = self.result_array((nch, nb, n0), np.float64)   # pinned when large: async copies
+        cs = None
+        if chan_scale is not None:
+            cs = np.ascontiguousarray(chan_scale, dtype=np.float64)
+            if cs.shape != (nch,):
+                raise ValueError("cwt_batch_products: one channel factor per channel expected")
+        want, fac, iw = 0, 0j, None
+        if icwt_factor is not None:
+            fac = complex(icwt_factor)
+            want = 2 if np.iscomplexobj(icwt_factor) else 1
+            iw = self.result_array((nch, n0), np.complex128 if want == 2 else np.float64)
+        with self.lock:
+            self._check(self.lib.cwtb_cwt_batch_products(
+                self.h, _ptr(X), int(X.dtype == np.float32), nch, n0, float(dt), _ptr(sj), sj.size,
+                int(family), float(param), int(precision),
+                _ptr(lo) if lo is not None else None, _ptr(hi) if hi is not None else None,
+                nb, _ptr(wt) if nb else None, _ptr(cs) if cs is not None else None,
+                fac.real, fac.imag, want, _ptr(power),
+                _ptr(power_coi) if power_coi is not None else None,
+                _ptr(band) if band is not None else None, _ptr(iw) if iw is not None else None))
+            self._resident = None                   # the last chunk of channels only
+        return power, power_coi, band, iw
 
     # ---- device-resident benchmarking helpers -------------------------------------
     @_locked

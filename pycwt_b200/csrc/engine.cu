@@ -234,6 +234,9 @@ struct cwtb_ctx {
   void *stage_host[2] = {nullptr, nullptr};
   size_t stage_bytes = 0;
   Buf stage_dev[2], batch_power;
+  // cwtb_cwt_batch_products: per-row COI sums of all chunks, the call's row / channel tables, and two
+  // device buffers of column outputs (chunk k writes one while the copy of chunk k-1 drains the other)
+  Buf batch_coi, prod_tab, prod_col[2];
   int batch_pipeline = 1;        // CWTB_BATCH_PIPELINE=0: one synchronous chunk after the other
   double *angle_host = nullptr;  // cwtb_wct: host destination of the phase angle, copied on a copy stream
                                  // as soon as it exists (before the smoothing transforms), not after them
@@ -257,6 +260,7 @@ struct cwtb_ctx {
   cudaEvent_t e0{}, e1{};
   cudaEvent_t ev_fork{}, ev_join{}, ev_joinc[3]{}, ev_coarse{};
   cudaEvent_t ev_h2d[2]{}, ev_used[2]{};
+  cudaEvent_t ev_prod[2]{}, ev_out[2]{};   // column outputs of a chunk written / copied to the host
   cudaEvent_t ev_xband{}, ev_pj[7]{}, ev_angle{};
 #endif
 };
@@ -1857,6 +1861,8 @@ int cwtb_create(int device, cwtb_ctx **out) {
   cudaEventCreateWithFlags(&c->ev_coarse, cudaEventDisableTiming);
   for (auto &ev : c->ev_h2d) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
   for (auto &ev : c->ev_used) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+  for (auto &ev : c->ev_prod) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+  for (auto &ev : c->ev_out) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
   if (const char *g = getenv("CWTB_BATCH_PIPELINE")) c->batch_pipeline = atoi(g) != 0;
   if (const char *g = getenv("CWTB_PRIO")) c->prio_mode = std::min(2, std::max(0, atoi(g)));
   for (auto &st : c->chain_streams) cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
@@ -1912,7 +1918,7 @@ void cwtb_destroy(cwtb_ctx *c) {
   cudaStreamSynchronize(c->stream);
 #endif
   cwtb_comm_destroy(c);
-  for (Buf *b : {&c->Zxs[0], &c->Zxs[1], &c->Zxs[2], &c->Zxs[3], &c->Zxs[4], &c->Zxs[5], &c->Zxs[6], &c->stage_dev[0], &c->stage_dev[1], &c->batch_power, &c->filt, &c->comm_send, &c->comm_recv, &c->Zx, &c->Cin, &c->Cout, &c->wtab, &c->ctr, &c->sig, &c->sig2, &c->spec, &c->Z, &c->Zc[0], &c->Zc[1], &c->Zc[2], &c->Y, &c->B, &c->W, &c->W2, &c->descs, &c->table, &c->scratch,
+  for (Buf *b : {&c->Zxs[0], &c->Zxs[1], &c->Zxs[2], &c->Zxs[3], &c->Zxs[4], &c->Zxs[5], &c->Zxs[6], &c->stage_dev[0], &c->stage_dev[1], &c->batch_power, &c->batch_coi, &c->prod_tab, &c->prod_col[0], &c->prod_col[1], &c->filt, &c->comm_send, &c->comm_recv, &c->Zx, &c->Cin, &c->Cout, &c->wtab, &c->ctr, &c->sig, &c->sig2, &c->spec, &c->Z, &c->Zc[0], &c->Zc[1], &c->Zc[2], &c->Y, &c->B, &c->W, &c->W2, &c->descs, &c->table, &c->scratch,
                  &c->C, &c->A12, &c->F, &c->aux, &c->rowd, &c->win, &c->mask, &c->hist, &c->noise, &c->wide, &c->blueA, &c->blueX, &c->blueY})
     if (b->p) rt_free(b->p);
   for (auto &kv : c->ntabs) { rt_free(kv.second.hi); rt_free(kv.second.lo); }
@@ -1935,6 +1941,8 @@ void cwtb_destroy(cwtb_ctx *c) {
   cudaEventDestroy(c->ev_coarse);
   for (auto &ev : c->ev_h2d) cudaEventDestroy(ev);
   for (auto &ev : c->ev_used) cudaEventDestroy(ev);
+  for (auto &ev : c->ev_prod) cudaEventDestroy(ev);
+  for (auto &ev : c->ev_out) cudaEventDestroy(ev);
   for (void *p : c->stage_host) if (p) cudaFreeHost(p);
   for (auto &st : c->chain_streams) cudaStreamDestroy(st);
   for (auto &ev : c->ev_joinc) cudaEventDestroy(ev);
@@ -2835,6 +2843,59 @@ int cwtb_profile_end(cwtb_ctx *c, char *out, size_t cap) {
 
 // Batched transform of independent channels: chunks of channels share every kernel launch
 // (one descriptor row per (channel, scale)).  X: host [n_chan][n0].
+
+// What a cwtb_cwt_batch_products call wants of every chunk: device tables, the per-row COI sums
+// and the host destinations of the column outputs.  A chunk of nc channels writes its columns to
+// one device buffer as [nc][nb][n0] band powers followed by [nc][n0][icw] icwt values.
+struct BatchProd {
+  int nb = 0, nbk = 2;          // bands in use; band accumulators of the kernel (2 or 8)
+  int icw = 0;                  // icwt doubles per column: 0 (none), 1 (real), 2 (complex)
+  double fre = 0, fim = 0;      // icwt factor
+  long long n0 = 0;
+  const double *wt = nullptr, *invs = nullptr, *cscale = nullptr;   // device [nbk][S], [S], [n_chan]
+  const long long *lo = nullptr, *hi = nullptr;                      // device [S], or null
+  double *dcoi = nullptr;       // device [n_chan][S] COI row sums, or null
+  double *band_out = nullptr, *icwt_out = nullptr;                   // host
+  size_t col_doubles(int nc) const { return (size_t)nc * (nb + icw) * n0; }
+};
+
+extern "C++" {   // (inside the C-ABI block)
+template <typename T, int NB>
+static int launch_products_t(cwtb_ctx *c, const BatchProd &p, int ch0, int nc, double *dcol, double *dsum) {
+  using B = BatchProductsBody<T, NB>;
+  const Job &job = c->job;
+  const int S = job.S;
+  const unsigned gx = (unsigned)((p.n0 + B::TILE - 1) / B::TILE);
+  for (int j0 = 0; j0 < S; j0 += B::RMAX) {
+    BatchProductsArgs<T> a{(const cx<T> *)c->W.p, p.wt, p.invs, p.lo, p.hi,
+                           p.cscale ? p.cscale + ch0 : nullptr, dsum, p.dcoi ? p.dcoi + (size_t)ch0 * S : nullptr,
+                           p.nb ? dcol : nullptr, p.icw ? dcol + (size_t)nc * p.nb * p.n0 : nullptr,
+                           p.fre, p.fim, p.n0, S, p.nb, p.icw == 2, j0, std::min(S, j0 + B::RMAX), j0 > 0};
+    if (int e = launch<B>(c, gx, (unsigned)nc, a)) return e;
+  }
+  return 0;
+}
+}
+
+// Products of the resident chunk (channels ch0 .. ch0+nc-1) on the engine's stream, no
+// synchronisation: row sums into dsum [nc][S] (and p.dcoi), column outputs into dcol.
+static int launch_batch_products(cwtb_ctx *c, const BatchProd &p, int ch0, int nc, double *dcol, double *dsum) {
+  if (c->job.precision == CWTB_F64)
+    return p.nbk == 2 ? launch_products_t<double, 2>(c, p, ch0, nc, dcol, dsum)
+                      : launch_products_t<double, 8>(c, p, ch0, nc, dcol, dsum);
+  return p.nbk == 2 ? launch_products_t<float, 2>(c, p, ch0, nc, dcol, dsum)
+                    : launch_products_t<float, 8>(c, p, ch0, nc, dcol, dsum);
+}
+
+// Column outputs of a chunk from dcol to the caller's arrays, on stream st.
+static int copy_batch_products(cwtb_ctx *c, const BatchProd &p, int ch0, int nc, const double *dcol, rt_stream st) {
+  const size_t nband = (size_t)nc * p.nb * p.n0;
+  if (p.nb) RT(rt_d2h(p.band_out + (size_t)ch0 * p.nb * p.n0, dcol, nband * sizeof(double), st));
+  if (p.icw)
+    RT(rt_d2h(p.icwt_out + (size_t)ch0 * p.icw * p.n0, dcol + nband, (size_t)nc * p.icw * p.n0 * sizeof(double), st));
+  return 0;
+}
+
 #ifndef CWTB_HOST_EMU
 // Per-row sums of |W|^2 of the resident chunk into dsum (device, R doubles, zeroed by the caller), on
 // the engine's stream, no synchronisation.
@@ -2852,9 +2913,12 @@ static int launch_row_power(cwtb_ctx *c, double *dsum) {
 
 // Spectra-only batch: chunk k+1 is copied into page-locked memory and sent to the device while the
 // kernels of chunk k run; nothing synchronises until the per-row power of all chunks is read back.
+// With `pr` (cwtb_cwt_batch_products) the products kernel takes the place of the row-power kernel;
+// the column outputs of chunk k go to device buffer k & 1, whose copy to the host is issued after
+// the kernels of chunk k+1 are queued, so it overlaps them.
 static int cwt_batch_pipelined(cwtb_ctx *c, const void *X, int x_is_f32, int n_chan, int64_t n0, double dt,
                                const double *scales, int n_scales, int family, double param, int precision,
-                               double *power_out, int nb) {
+                               double *power_out, int nb, const BatchProd *pr = nullptr) {
   const bool f32 = (precision == CWTB_F32);
   const size_t esz_in = x_is_f32 ? 4 : 8, esz = f32 ? 4 : 8;
   const size_t chunk_bytes = (size_t)nb * n0 * esz;
@@ -2873,10 +2937,14 @@ static int cwt_batch_pipelined(cwtb_ctx *c, const void *X, int x_is_f32, int n_c
   if ((e = ensure(c, c->batch_power, (size_t)n_chan * n_scales * sizeof(double)))) return e;
   double *dpow = (double *)c->batch_power.p;
   rt_stream copy = c->copy_streams[0];
+  rt_stream copy_out = c->copy_streams[1];   // the other direction: column outputs to the host
+  if (pr)
+    for (auto &b : c->prod_col)
+      if ((e = ensure(c, b, std::max<size_t>(1, pr->col_doubles(nb)) * sizeof(double)))) return e;
   RT(rt_memset(dpow, 0, (size_t)n_chan * n_scales * sizeof(double), c->stream));
   c->launches = 0;
   bool timing = false;
-  int k = 0;
+  int k = 0, prev_ch0 = 0, prev_nc = 0;
   for (int ch0 = 0; ch0 < n_chan; ch0 += nb, ++k) {
     const int nc = std::min(nb, n_chan - ch0), slot = k & 1;
     // (re-plans only when the chunk geometry changes: first and a shorter last chunk)
@@ -2903,13 +2971,34 @@ static int cwt_batch_pipelined(cwtb_ctx *c, const void *X, int x_is_f32, int n_c
     e = f32 ? run_job<float>(c, c->job, (const float *)c->stage_dev[slot].p)
             : run_job<double>(c, c->job, (const double *)c->stage_dev[slot].p);
     if (e) return e;
-    if ((e = launch_row_power(c, dpow + (size_t)ch0 * n_scales))) return e;
+    if (!pr) {
+      if ((e = launch_row_power(c, dpow + (size_t)ch0 * n_scales))) return e;
+    } else {
+      if (k >= 2) RT(cudaStreamWaitEvent(c->stream, c->ev_out[slot], 0));   // chunk k-2's columns are out
+      if ((e = launch_batch_products(c, *pr, ch0, nc, (double *)c->prod_col[slot].p, dpow + (size_t)ch0 * n_scales)))
+        return e;
+      RT(cudaEventRecord(c->ev_prod[slot], c->stream));
+      if (k >= 1) {   // chunk k-1's columns: copied while the kernels of chunk k run
+        RT(cudaStreamWaitEvent(copy_out, c->ev_prod[slot ^ 1], 0));
+        if ((e = copy_batch_products(c, *pr, prev_ch0, prev_nc, (const double *)c->prod_col[slot ^ 1].p, copy_out)))
+          return e;
+        RT(cudaEventRecord(c->ev_out[slot ^ 1], copy_out));
+      }
+      prev_ch0 = ch0;
+      prev_nc = nc;
+    }
     RT(cudaEventRecord(c->ev_used[slot], c->stream));
   }
   RT(cudaEventRecord(c->e1, c->stream));
+  if (pr) {
+    const int slot = (k - 1) & 1;
+    RT(cudaStreamWaitEvent(copy_out, c->ev_prod[slot], 0));
+    if ((e = copy_batch_products(c, *pr, prev_ch0, prev_nc, (const double *)c->prod_col[slot].p, copy_out))) return e;
+  }
   RT(rt_d2h(power_out, dpow, (size_t)n_chan * n_scales * sizeof(double), c->stream));
   RT(rt_sync(c->stream));
   RT(rt_sync(copy));
+  if (pr) RT(rt_sync(copy_out));
   float ms = 0;
   RT(cudaEventElapsedTime(&ms, c->e0, c->e1));
   c->last_ms = ms;
@@ -2956,6 +3045,128 @@ int cwtb_cwt_batch(cwtb_ctx *c, const void *X, int x_is_f32, int n_chan, int64_t
     if ((e = timed_run(c, c->sig.p, 1, &c->last_ms))) return e;
     if (power_out && (e = cwtb_global_power(c, power_out + (size_t)ch0 * n_scales))) return e;
     if (W_out && (e = cwtb_get_w(c, (char *)W_out + (size_t)ch0 * per_chan, 0, 0, nc * n_scales))) return e;
+  }
+  return 0;
+}
+
+int cwtb_cwt_batch_products(cwtb_ctx *c, const void *X, int x_is_f32, int n_chan, int64_t n0, double dt,
+                            const double *scales, int n_scales, int family, double param, int precision,
+                            const int64_t *coi_lo, const int64_t *coi_hi, int n_bands, const double *band_weights,
+                            const double *chan_scale, double icwt_re, double icwt_im, int want_icwt,
+                            double *power_out, double *power_coi_out, double *band_out, double *icwt_out) {
+  if (!c) return CWTB_ERR_ARG;
+  if (!X || !scales || !power_out || n_chan < 1 || n0 < 1 || n_scales < 1)
+    return fail(c, CWTB_ERR_ARG, "cwt_batch_products: bad argument");
+  if (n_bands < 0 || n_bands > 8) return fail(c, CWTB_ERR_ARG, "cwt_batch_products: n_bands must be 0..8");
+  if (n_bands > 0 && (!band_weights || !band_out))
+    return fail(c, CWTB_ERR_ARG, "cwt_batch_products: bands need band_weights and band_out");
+  if (!coi_lo != !coi_hi) return fail(c, CWTB_ERR_ARG, "cwt_batch_products: coi_lo and coi_hi go together");
+  if (!coi_lo != !power_coi_out) return fail(c, CWTB_ERR_ARG, "cwt_batch_products: COI ranges need power_coi_out");
+  if (want_icwt < 0 || want_icwt > 2 || (want_icwt && !icwt_out))
+    return fail(c, CWTB_ERR_ARG, "cwt_batch_products: want_icwt is 0, 1 (real) or 2 (complex) with icwt_out");
+  if (family == CWTB_TABLE) return fail(c, CWTB_ERR_UNSUPPORTED, "cwt_batch needs an analytic wavelet family");
+  if (!c->pad_pow2 && (n0 & (n0 - 1)) != 0) return fail(c, CWTB_ERR_UNSUPPORTED, "batched transforms need the padded mode");
+  const bool f32 = (precision == CWTB_F32);
+  const size_t esz_in = x_is_f32 ? 4 : 8, esz = f32 ? 4 : 8;
+  const int S = n_scales;
+  // channels per chunk as in cwtb_cwt_batch: coefficients of a chunk <= batch_bytes, rows <= 32768
+  const size_t per_chan = (f32 ? 8 : 16) * (size_t)n0 * S;
+  int nb = (int)std::max<size_t>(1, std::min<size_t>(c->batch_bytes / std::max<size_t>(per_chan, 1), 32768 / S));
+  nb = std::max(1, std::min(nb, n_chan));
+
+  // device tables: band weights [nbk][S] (zero rows past n_bands), 1/sqrt(s_j) [S], COI ranges
+  // [S] + [S] (int64), channel factors [n_chan]
+  BatchProd pr;
+  pr.nb = n_bands;
+  pr.nbk = n_bands <= 2 ? 2 : 8;
+  pr.icw = want_icwt;
+  pr.fre = icwt_re;
+  pr.fim = icwt_im;
+  pr.n0 = n0;
+  pr.band_out = band_out;
+  pr.icwt_out = icwt_out;
+  std::vector<double> tab((size_t)(pr.nbk + 3) * S + n_chan, 0.0);
+  for (int b = 0; b < n_bands; ++b)
+    for (int j = 0; j < S; ++j) tab[(size_t)b * S + j] = band_weights[(size_t)b * S + j];
+  double *t_invs = tab.data() + (size_t)pr.nbk * S;
+  for (int j = 0; j < S; ++j) t_invs[j] = 1.0 / std::sqrt(scales[j]);
+  std::vector<long long> cnt;
+  if (coi_lo) {
+    cnt.resize(S);
+    long long *t_lo = (long long *)(t_invs + S), *t_hi = t_lo + S;
+    for (int j = 0; j < S; ++j) {
+      t_lo[j] = std::max<long long>(0, coi_lo[j]);
+      t_hi[j] = std::min<long long>(n0, coi_hi[j]);
+      cnt[j] = t_hi[j] - t_lo[j];
+    }
+  }
+  double *t_cs = t_invs + 3 * (size_t)S;
+  for (int ch = 0; ch < n_chan; ++ch) t_cs[ch] = chan_scale ? chan_scale[ch] : 1.0;
+  int e = upload_doubles(c, c->prod_tab, tab);
+  if (e) return e;
+  const double *d_tab = (const double *)c->prod_tab.p;
+  pr.wt = d_tab;
+  pr.invs = d_tab + (size_t)pr.nbk * S;
+  if (coi_lo) {
+    pr.lo = (const long long *)(pr.invs + S);
+    pr.hi = pr.lo + S;
+  }
+  pr.cscale = chan_scale ? pr.invs + 3 * (size_t)S : nullptr;
+  const size_t rows_bytes = (size_t)n_chan * S * sizeof(double);
+  if (coi_lo) {
+    if ((e = ensure(c, c->batch_coi, rows_bytes))) return e;
+    pr.dcoi = (double *)c->batch_coi.p;
+    RT(rt_memset(pr.dcoi, 0, rows_bytes, c->stream));
+  }
+
+#ifndef CWTB_HOST_EMU
+  if (c->batch_pipeline) {
+    e = cwt_batch_pipelined(c, X, x_is_f32, n_chan, n0, dt, scales, n_scales, family, param, precision, power_out, nb, &pr);
+    if (e) return e;
+  } else
+#endif
+  {
+    // one chunk after the other: transform, products, copy, synchronise
+    if ((e = ensure(c, c->batch_power, rows_bytes))) return e;
+    if ((e = ensure(c, c->prod_col[0], std::max<size_t>(1, pr.col_doubles(nb)) * sizeof(double)))) return e;
+    double *dsum = (double *)c->batch_power.p;
+    RT(rt_memset(dsum, 0, rows_bytes, c->stream));
+    std::vector<unsigned char> conv;
+    for (int ch0 = 0; ch0 < n_chan; ch0 += nb) {
+      const int nc = std::min(nb, n_chan - ch0);
+      if ((e = prepare(c, n0, dt, scales, n_scales, family, param, precision, nullptr, nc))) return e;
+      if ((e = ensure(c, c->sig, (size_t)nc * n0 * esz))) return e;
+      const char *src = (const char *)X + (size_t)ch0 * n0 * esz_in;
+      if ((x_is_f32 != 0) == f32) {
+        RT(rt_h2d(c->sig.p, src, (size_t)nc * n0 * esz, c->stream));
+      } else {
+        conv.resize((size_t)nc * n0 * esz);
+        const size_t cnt_in = (size_t)nc * n0;
+        if (f32) for (size_t i = 0; i < cnt_in; ++i) ((float *)conv.data())[i] = (float)((const double *)src)[i];
+        else for (size_t i = 0; i < cnt_in; ++i) ((double *)conv.data())[i] = (double)((const float *)src)[i];
+        RT(rt_h2d(c->sig.p, conv.data(), conv.size(), c->stream));
+      }
+      RT(rt_sync(c->stream));
+      c->job_dsig = c->sig.p;
+      c->job.sig_is_f32 = f32;
+      if ((e = timed_run(c, c->sig.p, 1, &c->last_ms))) return e;
+      double *dcol = (double *)c->prod_col[0].p;
+      if ((e = launch_batch_products(c, pr, ch0, nc, dcol, dsum + (size_t)ch0 * S))) return e;
+      if ((e = copy_batch_products(c, pr, ch0, nc, dcol, c->stream))) return e;
+      RT(rt_sync(c->stream));
+    }
+    RT(rt_d2h(power_out, dsum, rows_bytes, c->stream));
+    RT(rt_sync(c->stream));
+    for (size_t i = 0; i < (size_t)n_chan * S; ++i) power_out[i] /= (double)n0;
+  }
+  if (coi_lo) {
+    RT(rt_d2h(power_coi_out, pr.dcoi, rows_bytes, c->stream));
+    RT(rt_sync(c->stream));
+    for (int ch = 0; ch < n_chan; ++ch)
+      for (int j = 0; j < S; ++j) {
+        double &v = power_coi_out[(size_t)ch * S + j];
+        v = cnt[j] > 0 ? v / (double)cnt[j] : std::nan("");
+      }
   }
   return 0;
 }

@@ -1538,6 +1538,148 @@ template <typename T> struct ScaleAvgBody {
   }
 };
 
+// ---- Body: per-channel products of a resident batch chunk W[nc][S][n] in one read ----------
+// For every channel c (blockIdx.y) and rows j0 <= j < j1 (simple_sample.py lines in brackets):
+//   rowsum[c][j]     += sum_n |W|^2                      (global spectrum before / n, :79)
+//   rowsum_coi[c][j] += sum_{lo_j <= n < hi_j} |W|^2     (the same inside the COI)
+//   band[c][b][n]    (+)= chan_scale[c] * sum_j wt[b][j] |W[c,j,n]|^2   (scale_avg, :88-91)
+//   isum[c][n]       (+)= fac * sum_j Re(W[c,j,n]) / sqrt(s_j)          (iwave, :60; complex fac:
+//                         isum[c][n][2] = (re, im))
+// One CTA owns a tile of TILE columns of one channel across all rows of the launch, so the
+// column outputs are written once by one thread, without atomics (bit-identical run to run).
+// The row sums are reduced in the warp, then in shared memory, and leave the CTA as one atomic
+// per row (PowerBody's note: per-warp atomics on one row address cost as much as the read).
+// NB: band accumulators per column (the bands in use, nb <= NB, are a launch argument).
+template <typename T> struct BatchProductsArgs {
+  const cx<T> *W;              // [nc][S][n]
+  const double *wt;            // [NB][S] band weights (rows b >= nb are not read)
+  const double *inv_sqrt_s;    // [S]
+  const long long *lo, *hi;    // [S] COI column ranges, or null
+  const double *chan_scale;    // [nc] (chunk's first channel), or null (1)
+  double *rowsum, *rowsum_coi; // [nc][S] (chunk's first channel); rowsum_coi null without ranges
+  double *band;                // [nc][nb][n], or null
+  double *isum;                // [nc][n] (icplx 0) or [nc][n][2] (icplx 1), or null
+  double fre, fim;             // icwt factor dj sqrt(dt) / (Cdelta psi(0))
+  long long n;
+  int S, nb, icplx;
+  int j0, j1, accumulate;      // rows of this launch (<= RMAX); accumulate: add to the column outputs
+};
+template <typename T, int NB> struct BatchProductsBody {
+  using Args = BatchProductsArgs<T>;
+  static constexpr int NPHASE = 3;
+  static constexpr int NTB = 256, CPT = 8, TILE = NTB * CPT;   // 2048 columns per CTA
+  static constexpr int U = sizeof(T) == 4 && NB <= 2 ? 2 : 1;  // rows per step: 16 loads of 8 B or 8 of 16 B in flight
+  static constexpr int MINB = NB <= 2 ? 2 : 1;                 // 8 bands: 72 accumulators per thread
+  static constexpr int RMAX = 1024;                            // rows per launch (shared row sums)
+  static constexpr size_t SMEM = 2 * RMAX * sizeof(double);
+  template <int PH> HD static void phase(const Args &a, int bx, int by, int tid, void *smraw) {
+    double *srow = (double *)smraw, *scoi = srow + RMAX;
+    const int nr = a.j1 - a.j0;
+    if constexpr (PH == 0) {
+      for (int r = tid; r < nr; r += NTB) { srow[r] = 0; scoi[r] = 0; }
+    } else if constexpr (PH == 1) {
+      const int nbase = bx * TILE + tid, ncol = (int)a.n;   // (32-bit columns: n < 2^28)
+      const cx<T> *Wc = a.W + (size_t)by * a.S * a.n;
+      double bacc[NB][CPT], iacc[CPT];
+#pragma unroll
+      for (int i = 0; i < CPT; ++i) {
+        iacc[i] = 0;
+#pragma unroll
+        for (int b = 0; b < NB; ++b) bacc[b][i] = 0;
+      }
+      for (int j = a.j0; j < a.j1; j += U) {
+        cx<T> w[U][CPT];
+        const cx<T> *row = Wc + (size_t)j * a.n + nbase;
+#pragma unroll
+        for (int u = 0; u < U; ++u)
+#pragma unroll
+          for (int i = 0; i < CPT; ++i)
+            w[u][i] = (j + u < a.j1 && nbase + i * NTB < ncol) ? ldg(&row[(size_t)u * a.n + i * NTB]) : mk<T>(0, 0);
+        double part[2 * U];   // row sum, COI row sum of each row of the step (this thread's columns)
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+          const int jr = j + u < a.j1 ? j + u : a.j1 - 1;   // rows past the end hold zeros
+          const double is = ldg(&a.inv_sqrt_s[jr]);
+          double wb[NB];
+#pragma unroll
+          for (int b = 0; b < NB; ++b) wb[b] = b < a.nb ? ldg(&a.wt[(size_t)b * a.S + jr]) : 0.0;
+          const int lo = a.lo ? (int)ldg(&a.lo[jr]) : 0, hi = a.lo ? (int)ldg(&a.hi[jr]) : 0;
+          double rs = 0, rc = 0;
+#pragma unroll
+          for (int i = 0; i < CPT; ++i) {
+            const int n = nbase + i * NTB;
+            const double x = (double)w[u][i].x, y = (double)w[u][i].y;
+            const double p = x * x + y * y;
+            rs += p;
+            rc += (n >= lo && n < hi) ? p : 0.0;
+#pragma unroll
+            for (int b = 0; b < NB; ++b) bacc[b][i] += wb[b] * p;
+            iacc[i] += x * is;
+          }
+          part[2 * u] = rs;
+          part[2 * u + 1] = rc;
+        }
+#if defined(__CUDA_ARCH__) && !defined(CWTB_HOST_EMU)
+        // 2U sums over the warp in (2U - 1) + (5 - log2 2U) shuffles: each halving step trades half
+        // of the values with the partner lane, so lane l ends with the total of value l % 2U
+        const int lane = tid & 31;
+#pragma unroll
+        for (int h = U; h >= 1; h >>= 1) {
+          const bool up = (lane & h) != 0;
+#pragma unroll
+          for (int v = 0; v < h; ++v) {
+            const double send = up ? part[v] : part[v + h];
+            const double keep = up ? part[v + h] : part[v];
+            part[v] = keep + __shfl_xor_sync(0xffffffffu, send, h);
+          }
+        }
+#pragma unroll
+        for (int o = 2 * U; o < 32; o <<= 1) part[0] += __shfl_xor_sync(0xffffffffu, part[0], o);
+        if (lane < 2 * U && j + lane / 2 < a.j1) atomicAdd(&((lane & 1) ? scoi : srow)[j + lane / 2 - a.j0], part[0]);
+#else
+#pragma unroll
+        for (int u = 0; u < U; ++u)
+          if (j + u < a.j1) { srow[j + u - a.j0] += part[2 * u]; scoi[j + u - a.j0] += part[2 * u + 1]; }
+#endif
+      }
+      const double cs = a.chan_scale ? a.chan_scale[by] : 1.0;
+#pragma unroll
+      for (int i = 0; i < CPT; ++i) {
+        const int n = nbase + i * NTB;
+        if (n >= ncol) continue;
+        if (a.band)
+#pragma unroll
+          for (int b = 0; b < NB; ++b) {
+            if (b >= a.nb) break;
+            double *o = &a.band[((size_t)by * a.nb + b) * a.n + n];
+            *o = a.accumulate ? *o + cs * bacc[b][i] : cs * bacc[b][i];
+          }
+        if (a.isum) {
+          if (a.icplx) {
+            double *o = &a.isum[((size_t)by * a.n + n) * 2];
+            o[0] = a.accumulate ? o[0] + a.fre * iacc[i] : a.fre * iacc[i];
+            o[1] = a.accumulate ? o[1] + a.fim * iacc[i] : a.fim * iacc[i];
+          } else {
+            double *o = &a.isum[(size_t)by * a.n + n];
+            *o = a.accumulate ? *o + a.fre * iacc[i] : a.fre * iacc[i];
+          }
+        }
+      }
+    } else {
+      for (int r = tid; r < nr; r += NTB) {
+        const size_t o = (size_t)by * a.S + a.j0 + r;
+#if defined(__CUDA_ARCH__) && !defined(CWTB_HOST_EMU)
+        atomicAdd(&a.rowsum[o], srow[r]);
+        if (a.rowsum_coi) atomicAdd(&a.rowsum_coi[o], scoi[r]);
+#else
+        a.rowsum[o] += srow[r];
+        if (a.rowsum_coi) a.rowsum_coi[o] += scoi[r];
+#endif
+      }
+    }
+  }
+};
+
 // ---- Body: real -> complex widening / complex -> real part ---------------------------------
 struct R2CArgs { const double *in; double2 *out; long long count; };
 struct R2CBody {

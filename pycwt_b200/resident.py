@@ -37,6 +37,28 @@ def _live(method):
     return wrapper
 
 
+def coi_ranges(wavelet, n0, dt, period):
+    """Columns inside the cone of influence of an n0-sample series, per period: period_j <= coi[n]
+    holds on one centred range [lo_j, hi_j) (empty ranges have lo_j == hi_j)."""
+    c = wavelet.flambda() * wavelet.coi() * dt
+    # coi[n] = c * (n0/2 - |n - (n0-1)/2|) >= period  <=>  |n - (n0-1)/2| <= n0/2 - period/c
+    half = n0 / 2 - np.asarray(period) / c
+    mid = (n0 - 1) / 2
+    lo = np.ceil(mid - half - 1e-12).astype(np.int64)
+    hi = np.floor(mid + half + 1e-12).astype(np.int64) + 1
+    empty = half < 0
+    lo = np.clip(lo, 0, n0)
+    hi = np.clip(hi, 0, n0)
+    hi[empty] = lo[empty]
+    return lo, hi
+
+
+def coi_curve(wavelet, n0, dt):
+    """The cone of influence of an n0-sample series, as `cwt` returns it (wavelet.py:118-120)."""
+    coi = (n0 / 2 - np.abs(np.arange(0, n0) - (n0 - 1) / 2))
+    return wavelet.flambda() * wavelet.coi() * dt * coi
+
+
 class ResidentTransform(object):
     """W[S, n0] of one `cwt_resident` call, resident on the device."""
 
@@ -58,9 +80,7 @@ class ResidentTransform(object):
     @property
     def coi(self):
         if self._coi is None:
-            n0 = self.n0
-            coi = (n0 / 2 - np.abs(np.arange(0, n0) - (n0 - 1) / 2))
-            self._coi = self.wavelet.flambda() * self.wavelet.coi() * self.dt * coi   # wavelet.py:118-120
+            self._coi = coi_curve(self.wavelet, self.n0, self.dt)
         return self._coi
 
     @property
@@ -110,18 +130,7 @@ class ResidentTransform(object):
     def coi_ranges(self):
         """Columns inside the cone of influence, per scale: period_j <= coi[n] holds on one
         centred range [lo_j, hi_j)."""
-        n0 = self.n0
-        c = self.wavelet.flambda() * self.wavelet.coi() * self.dt
-        # coi[n] = c * (n0/2 - |n - (n0-1)/2|) >= period  <=>  |n - (n0-1)/2| <= n0/2 - period/c
-        half = n0 / 2 - self.period / c
-        mid = (n0 - 1) / 2
-        lo = np.ceil(mid - half - 1e-12).astype(np.int64)
-        hi = np.floor(mid + half + 1e-12).astype(np.int64) + 1
-        empty = half < 0
-        lo = np.clip(lo, 0, n0)
-        hi = np.clip(hi, 0, n0)
-        hi[empty] = lo[empty]
-        return lo, hi
+        return coi_ranges(self.wavelet, self.n0, self.dt, self.period)
 
     @_live
     def global_power(self, inside_coi=False):
